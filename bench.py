@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K --warmup W    # the reference's CPU path on the host cores
     python bench.py --config c4                                       # NLMS_filter -> fast_xambg, 2M-sample CPI, 512 x 400
     python bench.py --config c5                                       # sweep CPI 256k..4M x Doppler 64..1024 (one line, "sweep": [...])
+    python bench.py --dump-outputs DIR                                # also write the maps of the last timed step to DIR
 
 One "step" = ``--frames-per-step`` CPI frames pushed through the frame pipeline: the rank's resident set of
 ``--resident`` DISTINCT frames (default 125 = BASELINE config 3's 1000-frame stream over 8 GPUs; 2.1 GB, far larger
@@ -71,7 +72,12 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stream", action="store_true", help="skip the config-3 NCCL staging measurement at N > 1")
     ap.add_argument("--cpu-procs", type=int, default=0, help="worker processes of the CPU arm (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the range-Doppler maps of the last timed step to DIR/*.npy (see dump_maps)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == "c5"):
+        ap.error("--dump-outputs writes the maps of the GPU arm of one configuration (not --impl reference or --config c5)")
+    return args
 
 
 def config_dict(cfg, args, world):
@@ -398,6 +404,25 @@ def make_resident(torch, dev, n, profile, count, rank, base=8):
     return ref_d, srv_d, np.stack(refs), np.stack(srvs)
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_maps(out_dir, maps_d, rank, world):
+    """Write the maps the last timed step computed (`maps_d`, one per resident frame it covered) so that two builds can be
+    compared map for map on the same seeded inputs: maps[.npy] = float32 (frames, F, R+1, 2) real/imaginary pairs, and
+    frame_index[.npy] = which resident frames they are (float64).  All frames when they fit in DUMP_BYTES over all ranks,
+    else a fixed seeded sample of frames.  With N > 1 each rank writes its own pair of files (suffix _rank<r>)."""
+    import torch
+    count = maps_d.shape[0]
+    keep = min(count, DUMP_BYTES // world // (maps_d[0].numel() * 8 + 8))
+    idx = np.arange(count) if keep == count else np.sort(np.random.default_rng(0).choice(count, keep, replace=False))
+    maps = torch.view_as_real(maps_d[torch.from_numpy(idx).to(maps_d.device)]).cpu().numpy()
+    suffix = f"_rank{rank}" if world > 1 else ""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"maps{suffix}.npy"), maps)
+    np.save(os.path.join(out_dir, f"frame_index{suffix}.npy"), idx.astype(np.float64))
+
+
 class Workload:
     """What one step runs, per config: c2/c1 the fused LS frame pipeline; c4 NLMS_filter (one CTA per frame, the batch
     fills the GPU) followed by the batched CAF of the cleaned channels."""
@@ -532,6 +557,9 @@ def run_b200(args, cfg, rank, world, local_rank, quiet=False):
     clocks = sampler.stop(t_begin, t_end) if rank == 0 else None
     frames_total = frames_per_step * args.steps * world
     value = frames_total / (ms * 1e-3)
+    if args.dump_outputs:
+        # a step walks the resident set from frame 0, so the last one wrote the maps of its first min(resident, frames) frames
+        dump_maps(args.dump_outputs, maps_d[:min(resident, frames_per_step)], rank, world)
 
     # ---- end to end through the public API with host buffers (pinned), copies inside the timed region
     nb_host = ref_base.shape[0]

@@ -7,6 +7,9 @@ import scipy.signal as signal
 from passiveradar_b200 import synth
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# OpenBLAS configuration the goldens were made with (make_golden.py sets it): complex64 matrix products of the
+# reference round differently with other kernels or thread counts
+GOLDEN_BLAS = {"OPENBLAS_CORETYPE": "SkylakeX", "OPENBLAS_NUM_THREADS": "8"}
 
 
 def load(name):

@@ -29,7 +29,10 @@ import os
 import sys
 import time
 
-import numpy as np
+# before numpy loads OpenBLAS: the goldens' BLAS configuration (tests/_golden.py GOLDEN_BLAS)
+os.environ.update(OPENBLAS_CORETYPE="SkylakeX", OPENBLAS_NUM_THREADS="8")
+
+import numpy as np  # noqa: E402
 import scipy.signal as signal
 
 HERE = os.path.dirname(os.path.abspath(__file__))

@@ -1,6 +1,10 @@
 """Pins the CPU oracle to the reference: every oracle function must reproduce the
 outputs the reference's own code produced (tests/golden/*.npz, made by
 tests/golden/make_golden.py with /root/reference on the path)."""
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 
@@ -35,11 +39,30 @@ def test_xambg_truth_formula_matches_reference(name):
     assert G.rel_inf(g["out"], truth) < 2e-6
 
 
+_LS_ORACLE_RUN = """
+import sys
+import numpy as np
+sys.path[:0] = sys.argv[1:3]
+import _golden as G
+from oracle import clutter_oracle as co
+g = G.load(sys.argv[3])
+ref, srv = G.inputs(g)
+out, taps = co.ls_filter_oracle(ref, srv, int(g["filter_len"]), float(g["reg"]), int(g["peek"]), True)
+np.savez(sys.argv[4], out=out, taps=taps)
+"""
+
+
 @pytest.mark.parametrize("name", G.LS_SMALL + G.LS_C1)
-def test_ls_oracle_matches_reference(name):
+def test_ls_oracle_matches_reference(name, tmp_path):
+    # the complex64 Gram of LS_Filter is one cgemm over n samples; its rounding depends on the BLAS kernels and thread
+    # count (up to 1e-5 in the taps of a 200k-sample frame), so the oracle runs with the BLAS the goldens were made with
+    res = tmp_path / "ls.npz"
+    tests_dir = os.path.dirname(os.path.abspath(__file__))
+    subprocess.run([sys.executable, "-c", _LS_ORACLE_RUN, tests_dir, os.path.dirname(tests_dir), name, str(res)],
+                   env=dict(os.environ, **G.GOLDEN_BLAS), check=True, timeout=600)
     g = G.load(name)
-    ref, srv = G.inputs(g)
-    out, taps = co.ls_filter_oracle(ref, srv, int(g["filter_len"]), float(g["reg"]), int(g["peek"]), True)
+    with np.load(res) as z:
+        out, taps = z["out"], z["taps"]
     assert out.dtype == np.complex64 and taps.dtype == np.complex64
     # BLAS threading may reorder the cgemm reduction between runs: allow float32 noise only
     assert G.rel_inf(taps, g["taps"]) < 2e-6
