@@ -242,6 +242,35 @@ int prc_frontend_c64(const void* in, int in_kind, int64_t n, int mode, double fc
 int prc_cfar2d_f32(const void* x, int rows, int cols, int fw, int gw, const float* thresh, float* cr_out,
                    uint8_t* det_out, int mem_kind, int device, void* stream, unsigned flags);
 
+/* ---- long-lag correlation and channel alignment (csrc/xcorr.cuh) -----------------------------------
+ * Replace xcorr() and find_channel_offset(), reference passiveRadar/signal_utils.py:29-78; main.py:54 and
+ * :83 call find_channel_offset(refc1, srvc1, 1, 5000000) once per run to align the two receiver channels.
+ * The correlation is a circular FP32 transform of P = 2^20 .. 2^24 points (four-step, float64-built
+ * twiddles); lag windows and inputs too long for one transform are tiled / segmented by the library.
+ *
+ * prc_xcorr_c64: xcorr(s1, s2, nlead, nlag) = scipy.signal.correlate(s1, np.pad(s2, (nlag, nlead)), 'valid')
+ *   is this lag window with, for L2 = ny + nlag + nlead, lag0 = ny - nx + nlead and nlags = L2 - nx + 1 when
+ *   L2 >= nx, else lag0 = -nlag and nlags = nx - L2 + 1.  nlags < 2^31.
+ *
+ * prc_channel_offset: B1, B2 = scipy.signal.decimate(s, nd) (zero-phase: sosfiltfilt with the caller's
+ *   sections, odd extension of 3 (2 nsections + 1) samples, sosfilt_zi initial states, float64 state), then
+ *   xc = |xcorr(B1, B2, nl, nl)| (|Re| for real inputs) and *offset = (argmax xc - nl) * nd, the first index
+ *   winning ties.  sos: nsections x 6 host doubles with sos[s][3] == 1 (scipy.signal.cheby1(8, 0.05, 0.8 / nd,
+ *   output='sos') for decimate's default filter).  in_kind: one PRC_SIG_* (real integers are upcast to
+ *   float64 as decimate does).  xc_abs: optional, receives the nlags floats of |xc| (2 nl + 1 when both
+ *   decimated channels have the same length).  offset is one int64 in memory of mem_kind.
+ */
+#define PRC_SIG_C64   0   /* complex64 samples */
+#define PRC_SIG_I8    1   /* real int8 samples (the raw arrays main.py:81-83 reads) */
+#define PRC_SIG_I16   2   /* real int16 samples */
+#define PRC_SIG_F64   3   /* real float64 samples */
+#define PRC_SIG_C128  4   /* complex128 samples */
+int prc_xcorr_c64(const prc_c64* x, int64_t nx, const prc_c64* y, int64_t ny, int64_t lag0, int64_t nlags,
+                  prc_c64* out, int mem_kind, int device, void* stream, unsigned flags);
+int prc_channel_offset(const void* s1, int64_t n1, const void* s2, int64_t n2, int in_kind, int nd, int64_t nl,
+                       const double* sos, int nsections, int64_t* offset, float* xc_abs,
+                       int mem_kind, int device, void* stream, unsigned flags);
+
 #ifdef __cplusplus
 }
 #endif

@@ -13,17 +13,19 @@ from .range_doppler_processing import fast_xambg, direct_xambg            # noqa
 from .clutter_removal import (LS_Filter, NLMS_filter, block_NLMS,            # noqa: F401
                               LS_Filter_Toeplitz, LS_Filter_Multiple)
 from .signal_utils import deinterleave_IQ, frequency_shift, resample, frontend            # noqa: F401
+from .signal_utils import xcorr, find_channel_offset, offset_compensation            # noqa: F401
 from .target_detection import CFAR_2D            # noqa: F401
 
 __all__ = ["fast_xambg", "direct_xambg", "LS_Filter", "NLMS_filter", "block_NLMS", "LS_Filter_Toeplitz",
-           "LS_Filter_Multiple", "deinterleave_IQ", "frequency_shift", "resample", "frontend", "CFAR_2D"]
+           "LS_Filter_Multiple", "deinterleave_IQ", "frequency_shift", "resample", "frontend", "CFAR_2D",
+           "xcorr", "find_channel_offset", "offset_compensation"]
 __version__ = "0.1.0"
 
 
 def install(reference_package: str = "passiveRadar"):
     """Swap the hot-path functions of an importable copy of the reference for the GPU ones.
 
-    ``main.py`` binds ``fast_xambg``, ``LS_Filter_Multiple`` and ``NLMS_filter`` with
+    ``main.py`` binds ``find_channel_offset``, ``fast_xambg``, ``LS_Filter_Multiple`` and ``NLMS_filter`` with
     ``from passiveRadar... import ...`` (main.py:10-14); calling ``install()`` before ``main.py`` is
     imported/run makes those names resolve to this package while config, I/O and the dask graph stay
     the reference's own code::
@@ -36,7 +38,8 @@ def install(reference_package: str = "passiveRadar"):
     replaced = []
     table = {
         "range_doppler_processing": {"fast_xambg": fast_xambg, "direct_xambg": direct_xambg},
-        "signal_utils": {"deinterleave_IQ": deinterleave_IQ, "frequency_shift": frequency_shift, "resample": resample},
+        "signal_utils": {"deinterleave_IQ": deinterleave_IQ, "frequency_shift": frequency_shift, "resample": resample,
+                         "find_channel_offset": find_channel_offset, "offset_compensation": offset_compensation},
         "target_detection": {"CFAR_2D": CFAR_2D},
         "clutter_removal": {"LS_Filter": LS_Filter, "NLMS_filter": NLMS_filter,
                             "LS_Filter_Toeplitz": LS_Filter_Toeplitz, "LS_Filter_Multiple": LS_Filter_Multiple},

@@ -28,6 +28,7 @@ FLAG_WINDOW_F32 = 2
 FLAG_ABS_C64 = 4
 IQ_C64, IQ_I8, IQ_I16 = 0, 1, 2
 MIX_NONE, MIX_C64, MIX_C128, MIX_F64, MIX_FS64 = 0, 1, 2, 3, 4
+SIG_C64, SIG_I8, SIG_I16, SIG_F64, SIG_C128 = 0, 1, 2, 3, 4
 
 # every symbol include/prcore.h declares: name -> (restype, argtypes)
 _c64p = C.c_void_p
@@ -81,6 +82,11 @@ SIGNATURES = {
                                    C.c_int, C.c_int, C.c_void_p, C.c_uint]),
     "prc_cfar2d_f32": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                  C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint]),
+    "prc_xcorr_c64": (C.c_int, [_c64p, C.c_int64, _c64p, C.c_int64, C.c_int64, C.c_int64, _c64p,
+                                C.c_int, C.c_int, C.c_void_p, C.c_uint]),
+    "prc_channel_offset": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int64,
+                                     C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                     C.c_int, C.c_int, C.c_void_p, C.c_uint]),
 }
 
 _lib = None

@@ -30,6 +30,7 @@
 #include "nlms.cuh"
 #include "nlms_block.cuh"
 #include "fftcorr.cuh"
+#include "xcorr.cuh"
 
 namespace {
 
@@ -52,9 +53,9 @@ thread_local std::string g_err;
 std::atomic<uint64_t> g_launches{0};
 
 // optional per-kernel timing (prc_profile_*): CUDA events on the launching stream around each launch
-enum KernelId { K_LAGCORR_LS = 0, K_LEVINSON, K_FIR, K_LAGCORR_CAF, K_DOPPLER, K_NLMS, K_MISC, K_COUNT };
+enum KernelId { K_LAGCORR_LS = 0, K_LEVINSON, K_FIR, K_LAGCORR_CAF, K_DOPPLER, K_NLMS, K_MISC, K_IIR, K_XCORR, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"lagcorr_ls", "levinson", "fir_apply", "lagcorr_caf",
-                                           "doppler_fft", "nlms", "misc"};
+                                           "doppler_fft", "nlms", "misc", "iir_sos", "xcorr_fft"};
 std::atomic<int> g_prof_on{0};
 std::mutex g_prof_mu;
 double g_prof_ms[K_COUNT] = {0};
@@ -138,6 +139,10 @@ struct Ctx {
     bool pin_ready = false;
     DBuf fft_tw[3], wp_fir, wp_caf, fftP;     // FFT-domain path: twiddle tables (L = 1024 / 2048 / 4096), taps spectra, CAF block sums
     bool fft_tw_ready[3] = {false, false, false};
+    // long-lag correlation / channel offset (xcorr.cuh): raw inputs, forward IIR pass, decimated channels,
+    // transform planes, W_P tables (for xc_twP), argmax key + offset, |xc| / lag window staging
+    DBuf xc_in1, xc_in2, xc_yf, xc_b1, xc_b2, xc_X, xc_Y, xc_S, xc_tw, xc_key, xc_out;
+    long long xc_twP = 0;
     std::vector<ProfRec> recs;
     void release() {
         cudaSetDevice(device);
@@ -149,6 +154,8 @@ struct Ctx {
         for (DBuf& b : fft_tw) b.release();
         for (bool& r : fft_tw_ready) r = false;
         for (DBuf* b : {&wp_fir, &wp_caf, &fftP}) b->release();
+        for (DBuf* b : {&xc_in1, &xc_in2, &xc_yf, &xc_b1, &xc_b2, &xc_X, &xc_Y, &xc_S, &xc_tw, &xc_key, &xc_out}) b->release();
+        xc_twP = 0;
         for (DBuf* b : {&fe_in, &fe_mid, &fe_out, &fe_hp, &fe_ends, &cf_in, &cf_cr, &cf_det, &cf_part}) b->release();
         for (DBuf* b : {&refw, &ref, &srv, &out, &clean, &partial, &win32, &win64, &dtaps32, &dtaps64, &lstaps,
                         &tw, &pbuf, &status, &nl_init, &nl_taps})
@@ -266,6 +273,17 @@ int set_kernel_attrs(int device) {
     PRC_FFT_ATTRS(8)
     PRC_FFT_ATTRS(16)
 #undef PRC_FFT_ATTRS
+#define PRC_XC_ATTRS(R1, R2)                                                                                           \
+    CU(cudaFuncSetAttribute(xc::col_fwd_kernel<R1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));                \
+    CU(cudaFuncSetAttribute(xc::col_inv_kernel<R1>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));                \
+    CU(cudaFuncSetAttribute(xc::row_fwd_kernel<R2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));                \
+    CU(cudaFuncSetAttribute(xc::row_prod_kernel<R1, R2>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+    PRC_XC_ATTRS(4, 4)
+    PRC_XC_ATTRS(8, 4)
+    PRC_XC_ATTRS(8, 8)
+    PRC_XC_ATTRS(16, 8)
+    PRC_XC_ATTRS(16, 16)
+#undef PRC_XC_ATTRS
     g_attrs_set[device].store(true);
     return PRC_OK;
 }
@@ -1556,6 +1574,210 @@ int frame_device(Ctx* c, const float2* ref, const float2* srv, long long n, Batc
 
 bool bad_mem_kind(int k) { return k != PRC_MEM_HOST && k != PRC_MEM_DEVICE; }
 
+// --------------------------------------------------------------------------- long-lag correlation (xcorr.cuh)
+// Tile plan: one circular transform of P = 2^20 .. 2^24 points holds Lseg x samples and nt lags without wrap-around
+// when Lseg + nt - 1 <= P.  Lag windows longer than that are cut into tiles, x into segments whose spectra are
+// accumulated before the transform back.
+struct XcPlan {
+    int r1 = 4, r2 = 4;
+    long long P = 0, seg = 0, tile = 0;
+    long long nseg = 0, ntile = 0;
+};
+
+constexpr long long XC_PMIN = 1ll << 20, XC_PMAX = 1ll << 24;
+
+XcPlan xc_plan(long long nx, long long nlags) {
+    XcPlan pl;
+    const long long need = nx + nlags - 1;
+    if (need <= XC_PMAX) {
+        pl.P = XC_PMIN;
+        while (pl.P < need) pl.P <<= 1;
+        pl.seg = nx;
+        pl.tile = nlags;
+    } else {
+        pl.P = XC_PMAX;
+        pl.tile = std::min(nlags, XC_PMAX / 2);
+        pl.seg = XC_PMAX - pl.tile + 1;
+        if (nx < pl.seg) {
+            pl.seg = nx;
+            pl.tile = XC_PMAX - nx + 1;
+        }
+    }
+    pl.nseg = (nx + pl.seg - 1) / pl.seg;
+    pl.ntile = (nlags + pl.tile - 1) / pl.tile;
+    // L1 x L2 = P, L1 >= L2
+    const int lg = ilog2((int)(pl.P >> 20));      // P = 2^20 .. 2^24
+    static const int r1s[5] = {4, 8, 8, 16, 16}, r2s[5] = {4, 4, 8, 8, 16};
+    pl.r1 = r1s[lg];
+    pl.r2 = r2s[lg];
+    return pl;
+}
+
+int xc_p_twiddles(Ctx* c, long long P, const float2** lo, const float2** hi) {
+    TRY(c->xc_tw.ensure(8192 * sizeof(float2)));
+    if (c->xc_twP != P) {
+        xc::p_twiddle_kernel<<<ceil_div(4096 + P / 4096, 256), 256, 0, c->stream>>>(c->xc_tw.as<float2>(),
+                                                                                   c->xc_tw.as<float2>() + 4096, P);
+        TRY(check_launch("p_twiddle_kernel"));
+        c->xc_twP = P;
+    }
+    *lo = c->xc_tw.as<float2>();
+    *hi = c->xc_tw.as<float2>() + 4096;
+    return PRC_OK;
+}
+
+// out[j] = sum_i x[i] conj(y[i + lag0 - j]), j < nlags (device pointers).  out: complex lags, absout: |xc| (|Re xc| when
+// real), best: argmax key (bits(|xc|) << 32 | ~j, max-reduced; caller zeroes it).  Any of the three may be NULL.
+int xcorr_device(Ctx* c, const float2* x, long long nx, const float2* y, long long ny, long long lag0, long long nlags,
+                 float2* out, float* absout, unsigned long long* best, bool real) {
+    const XcPlan pl = xc_plan(nx, nlags);
+    const int L1 = 256 * pl.r1, L2 = 256 * pl.r2;
+    const float2 *tw1, *tw2, *plo, *phi;
+    TRY(fft_twiddles(c, pl.r1, &tw1));
+    TRY(fft_twiddles(c, pl.r2, &tw2));
+    TRY(xc_p_twiddles(c, pl.P, &plo, &phi));
+    TRY(c->xc_X.ensure((size_t)pl.P * sizeof(float2)));
+    TRY(c->xc_Y.ensure((size_t)pl.P * sizeof(float2)));
+    if (pl.nseg > 1) TRY(c->xc_S.ensure((size_t)pl.P * sizeof(float2)));
+    float2* X = c->xc_X.as<float2>();
+    float2* Y = c->xc_Y.as<float2>();
+    const size_t sm1 = fft_smem(pl.r1), sm2 = fft_smem(pl.r2);
+    ProfScope ps(c, K_XCORR);
+    for (long long ti = 0; ti < pl.ntile; ++ti) {
+        const long long j0 = ti * pl.tile, nt = std::min(pl.tile, nlags - j0);
+        const long long m_lo = lag0 - j0 - nt + 1;
+        for (long long si = 0; si < pl.nseg; ++si) {
+            const long long s = si * pl.seg, ls = std::min(pl.seg, nx - s);
+            xc::ColFwdParams cp{};
+            cp.L2 = L2; cp.tw = tw1; cp.plo = plo; cp.phi = phi;
+            xc::RowParams rp{};
+            rp.L2 = L2; rp.tw = tw2; rp.plo = plo; rp.phi = phi;
+            // x segment -> X spectrum
+            cp.src = x; cp.off = s; cp.nsrc = nx; cp.lim = ls; cp.Z = X;
+            rp.Z = X;
+            PRC_R3_SWITCH(pl.r1, (xc::col_fwd_kernel<R3><<<L2 / xc::NCOL, 16 * R3, sm1, c->stream>>>(cp)));
+            TRY(check_launch("col_fwd_kernel"));
+            PRC_R3_SWITCH(pl.r2, (xc::row_fwd_kernel<R3><<<L1, 16 * R3, sm2, c->stream>>>(rp)));
+            TRY(check_launch("row_fwd_kernel"));
+            // the P samples of y that lags m_lo .. m_lo + nt - 1 of the segment reach -> product spectrum
+            cp.src = y; cp.off = s + m_lo; cp.nsrc = ny; cp.lim = pl.P; cp.Z = Y;
+            rp.Z = Y; rp.Xh = X; rp.S = c->xc_S.as<float2>();
+            rp.acc_in = si > 0; rp.last = si + 1 == pl.nseg;
+            PRC_R3_SWITCH(pl.r1, (xc::col_fwd_kernel<R3><<<L2 / xc::NCOL, 16 * R3, sm1, c->stream>>>(cp)));
+            TRY(check_launch("col_fwd_kernel"));
+            switch (pl.r1 * 100 + pl.r2) {
+                case 404: xc::row_prod_kernel<4, 4><<<L1, 64, sm2, c->stream>>>(rp); break;
+                case 804: xc::row_prod_kernel<8, 4><<<L1, 64, sm2, c->stream>>>(rp); break;
+                case 808: xc::row_prod_kernel<8, 8><<<L1, 128, sm2, c->stream>>>(rp); break;
+                case 1608: xc::row_prod_kernel<16, 8><<<L1, 128, sm2, c->stream>>>(rp); break;
+                default: xc::row_prod_kernel<16, 16><<<L1, 256, sm2, c->stream>>>(rp); break;
+            }
+            TRY(check_launch("row_prod_kernel"));
+        }
+        xc::ColInvParams ip{};
+        ip.Z = Y; ip.L2 = L2; ip.nt = nt; ip.j_hi = j0 + nt - 1;
+        ip.scale = 1.0f / (float)pl.P;
+        ip.out = out; ip.absout = absout; ip.best = best; ip.real = real ? 1 : 0;
+        ip.tw = tw1;
+        PRC_R3_SWITCH(pl.r1, (xc::col_inv_kernel<R3><<<L2 / xc::NCOL, 16 * R3, sm1, c->stream>>>(ip)));
+        TRY(check_launch("col_inv_kernel"));
+    }
+    return PRC_OK;
+}
+
+// scipy.signal.sosfiltfilt's filter as the device runs it: normalised sections, sosfilt_zi, padlen, warm-up length
+struct SosDesign {
+    int ns = 0, pad = 0, warm = 0;
+    double c[xc::SOS_MAX][5], zi[xc::SOS_MAX][2];
+};
+
+int sos_design(const double* sos, int nsec, SosDesign* d) {
+    if (!sos || nsec < 1 || nsec > xc::SOS_MAX) return fail(PRC_E_INVALID, "nsections=%d invalid (1..%d)", nsec, xc::SOS_MAX);
+    d->ns = nsec;
+    int zb = 0, za = 0;
+    double rho = 0.0, scale = 1.0;
+    for (int s = 0; s < nsec; ++s) {
+        const double* q = sos + 6 * s;
+        if (q[3] != 1.0) return fail(PRC_E_INVALID, "sos[%d, 3] must be 1", s);
+        zb += q[2] == 0.0;
+        za += q[5] == 0.0;
+        const double b0 = q[0], b1 = q[1], b2 = q[2], a1 = q[4], a2 = q[5];
+        d->c[s][0] = b0; d->c[s][1] = b1; d->c[s][2] = b2; d->c[s][3] = a1; d->c[s][4] = a2;
+        // lfilter_zi of the section: (I - companion(a)^T) zi = b[1:] - a[1:] b0
+        const double B0 = b1 - a1 * b0, B1 = b2 - a2 * b0;
+        const double den = 1.0 + a1 + a2;
+        if (den == 0.0) return fail(PRC_E_INVALID, "section %d has a pole at z = 1", s);
+        const double z0 = (B0 + B1) / den;
+        d->zi[s][0] = scale * z0;
+        d->zi[s][1] = scale * (B1 - a2 * z0);
+        scale *= (b0 + b1 + b2) / den;
+        // pole radius of z^2 + a1 z + a2
+        const double disc = a1 * a1 - 4.0 * a2;
+        const double r = disc < 0.0 ? std::sqrt(a2) : std::max(std::fabs(-a1 + std::sqrt(disc)), std::fabs(-a1 - std::sqrt(disc))) / 2.0;
+        rho = std::max(rho, r);
+    }
+    for (int s = nsec; s < xc::SOS_MAX; ++s)
+        for (int k = 0; k < 5; ++k) d->c[s][k] = 0.0, d->zi[s][k % 2] = 0.0;
+    if (!(rho < 1.0)) return fail(PRC_E_INVALID, "unstable filter (pole radius %.6f)", rho);
+    d->pad = 3 * (2 * nsec + 1 - std::min(zb, za));
+    // free response below 1e-20 of the state it forgets
+    d->warm = rho > 0.0 ? (int)std::min(1e7, std::ceil(std::log(1e-20) / std::log(rho))) : 0;
+    d->warm = std::max(d->warm, 32);
+    return PRC_OK;
+}
+
+size_t sig_elem(int kind) {
+    switch (kind) {
+        case xc::SIG_I8: return 1;
+        case xc::SIG_I16: return 2;
+        case xc::SIG_F64: return 8;
+        case xc::SIG_C64: return 8;
+        default: return 16;
+    }
+}
+bool sig_complex(int kind) { return kind == xc::SIG_C64 || kind == xc::SIG_C128; }
+
+// sosfiltfilt(sos, in)[::nd] -> out (complex64, ceil(n / nd) samples)
+int decimate_device(Ctx* c, const void* in, int kind, long long n, const SosDesign& d, int nd, float2* out) {
+    xc::IirParams p{};
+    p.in = in; p.kind = kind; p.n = n; p.ns = d.ns; p.pad = d.pad;
+    p.ne = n + 2ll * d.pad;
+    p.chunk = 1024; p.warm = d.warm;
+    memcpy(p.c, d.c, sizeof p.c);
+    memcpy(p.zi, d.zi, sizeof p.zi);
+    const bool cplx = sig_complex(kind);
+    TRY(c->xc_yf.ensure((size_t)p.ne * (cplx ? sizeof(double2) : sizeof(double))));
+    p.yf = c->xc_yf.p;
+    p.out = out; p.nd = nd; p.nout = (n + nd - 1) / nd;
+    const int nthr = ceil_div(p.ne, p.chunk);
+    ProfScope ps(c, K_IIR);
+    if (cplx) {
+        xc::iir_fwd_kernel<double2><<<ceil_div(nthr, 32), 32, 0, c->stream>>>(p);
+        TRY(check_launch("iir_fwd_kernel"));
+        xc::iir_bwd_kernel<double2><<<ceil_div(nthr, 32), 32, 0, c->stream>>>(p);
+    } else {
+        xc::iir_fwd_kernel<double><<<ceil_div(nthr, 32), 32, 0, c->stream>>>(p);
+        TRY(check_launch("iir_fwd_kernel"));
+        xc::iir_bwd_kernel<double><<<ceil_div(nthr, 32), 32, 0, c->stream>>>(p);
+    }
+    return check_launch("iir_bwd_kernel");
+}
+
+// lag window of scipy.signal.correlate(s1, np.pad(s2, (nlag, nlead)), 'valid') (reference signal_utils.py:29-32):
+// out[k] = c[lag0 - k], k < nlags
+void xcorr_window(long long n1, long long n2, long long nlead, long long nlag, long long* lag0, long long* nlags) {
+    const long long L2 = n2 + nlag + nlead;
+    if (L2 >= n1) {
+        *lag0 = n2 - n1 + nlead;
+        *nlags = L2 - n1 + 1;
+    } else {
+        *lag0 = -nlag;
+        *nlags = n1 - L2 + 1;
+    }
+}
+
+constexpr long long XC_MAX_LAGS = 0x7FFFFFFFll;    // lag indices fit the 32 low bits of the argmax key
+
 }  // namespace
 
 // =========================================================================== C ABI
@@ -2193,6 +2415,92 @@ int prc_direct_xambg_c64(const prc_c64* ref, const prc_c64* srv, int64_t n, int 
     }
     TRY(direct_xambg_device(c, dref, dsrv, n, range_bins, freq_bins, sample_rate, dout));
     if (mem_kind == PRC_MEM_HOST) TRY(d2h(c, out, dout, ob, flags));
+    return finish(c, flags);
+}
+
+}  // extern "C"
+
+extern "C" {
+
+int prc_xcorr_c64(const prc_c64* x, int64_t nx, const prc_c64* y, int64_t ny, int64_t lag0, int64_t nlags,
+                  prc_c64* out, int mem_kind, int device, void* stream, unsigned flags) {
+    if (!x || !y || !out) return fail(PRC_E_INVALID, "x/y/out must not be NULL");
+    if (bad_mem_kind(mem_kind)) return fail(PRC_E_INVALID, "mem_kind=%d invalid", mem_kind);
+    if (nx <= 0 || ny <= 0) return fail(PRC_E_INVALID, "nx=%lld / ny=%lld invalid", (long long)nx, (long long)ny);
+    if (nlags <= 0 || nlags > XC_MAX_LAGS) return fail(PRC_E_INVALID, "nlags=%lld invalid (1..%lld)", (long long)nlags, XC_MAX_LAGS);
+    Ctx* c;
+    TRY(get_ctx(device, stream, &c));
+    std::lock_guard<std::mutex> lk(c->mu);
+    const float2* dx = reinterpret_cast<const float2*>(x);
+    const float2* dy = reinterpret_cast<const float2*>(y);
+    float2* dout = reinterpret_cast<float2*>(out);
+    const size_t ob = (size_t)nlags * sizeof(float2);
+    if (mem_kind == PRC_MEM_HOST) {
+        TRY(c->xc_b1.ensure((size_t)nx * sizeof(float2)));
+        TRY(c->xc_b2.ensure((size_t)ny * sizeof(float2)));
+        TRY(c->xc_out.ensure(ob));
+        TRY(h2d(c, c->xc_b1.p, x, (size_t)nx * sizeof(float2), flags));
+        TRY(h2d(c, c->xc_b2.p, y, (size_t)ny * sizeof(float2), flags));
+        dx = c->xc_b1.as<float2>();
+        dy = c->xc_b2.as<float2>();
+        dout = c->xc_out.as<float2>();
+    }
+    TRY(xcorr_device(c, dx, nx, dy, ny, lag0, nlags, dout, nullptr, nullptr, false));
+    if (mem_kind == PRC_MEM_HOST) TRY(d2h(c, out, dout, ob, flags));
+    return finish(c, flags);
+}
+
+int prc_channel_offset(const void* s1, int64_t n1, const void* s2, int64_t n2, int in_kind, int nd, int64_t nl,
+                       const double* sos, int nsections, int64_t* offset, float* xc_abs,
+                       int mem_kind, int device, void* stream, unsigned flags) {
+    if (!s1 || !s2 || !offset) return fail(PRC_E_INVALID, "s1/s2/offset must not be NULL");
+    if (bad_mem_kind(mem_kind)) return fail(PRC_E_INVALID, "mem_kind=%d invalid", mem_kind);
+    if (in_kind < PRC_SIG_C64 || in_kind > PRC_SIG_C128) return fail(PRC_E_INVALID, "in_kind=%d invalid", in_kind);
+    if (nd < 1) return fail(PRC_E_INVALID, "nd=%d invalid", nd);
+    if (nl < 0) return fail(PRC_E_INVALID, "nl=%lld invalid", (long long)nl);
+    SosDesign d;
+    TRY(sos_design(sos, nsections, &d));
+    if (n1 <= d.pad || n2 <= d.pad)
+        return fail(PRC_E_INVALID, "n1=%lld / n2=%lld: the inputs must be longer than padlen=%d", (long long)n1, (long long)n2, d.pad);
+    const long long n1d = (n1 + nd - 1) / nd, n2d = (n2 + nd - 1) / nd;
+    long long lag0, nlags;
+    xcorr_window(n1d, n2d, nl, nl, &lag0, &nlags);
+    if (nlags > XC_MAX_LAGS) return fail(PRC_E_INVALID, "%lld lags exceed %lld", nlags, XC_MAX_LAGS);
+    Ctx* c;
+    TRY(get_ctx(device, stream, &c));
+    std::lock_guard<std::mutex> lk(c->mu);
+    const void* d1 = s1;
+    const void* d2 = s2;
+    if (mem_kind == PRC_MEM_HOST) {
+        const size_t b1 = (size_t)n1 * sig_elem(in_kind), b2 = (size_t)n2 * sig_elem(in_kind);
+        TRY(c->xc_in1.ensure(b1));
+        TRY(c->xc_in2.ensure(b2));
+        TRY(h2d(c, c->xc_in1.p, s1, b1, flags));
+        TRY(h2d(c, c->xc_in2.p, s2, b2, flags));
+        d1 = c->xc_in1.p;
+        d2 = c->xc_in2.p;
+    }
+    TRY(c->xc_b1.ensure((size_t)n1d * sizeof(float2)));
+    TRY(c->xc_b2.ensure((size_t)n2d * sizeof(float2)));
+    TRY(decimate_device(c, d1, in_kind, n1, d, nd, c->xc_b1.as<float2>()));
+    TRY(decimate_device(c, d2, in_kind, n2, d, nd, c->xc_b2.as<float2>()));
+    TRY(c->xc_key.ensure(2 * sizeof(unsigned long long)));
+    unsigned long long* key = c->xc_key.as<unsigned long long>();
+    CU(cudaMemsetAsync(key, 0, sizeof(unsigned long long), c->stream));
+    float* dabs = xc_abs;
+    if (xc_abs && mem_kind == PRC_MEM_HOST) {
+        TRY(c->xc_out.ensure((size_t)nlags * sizeof(float)));
+        dabs = c->xc_out.as<float>();
+    }
+    TRY(xcorr_device(c, c->xc_b1.as<float2>(), n1d, c->xc_b2.as<float2>(), n2d, lag0, nlags, nullptr, dabs, key,
+                     !sig_complex(in_kind)));
+    long long* doff = mem_kind == PRC_MEM_HOST ? reinterpret_cast<long long*>(key + 1) : reinterpret_cast<long long*>(offset);
+    xc::offset_kernel<<<1, 1, 0, c->stream>>>(key, nl, nd, doff);
+    TRY(check_launch("offset_kernel"));
+    if (mem_kind == PRC_MEM_HOST) {
+        if (xc_abs) TRY(d2h(c, xc_abs, dabs, (size_t)nlags * sizeof(float), flags));
+        CU(cudaMemcpyAsync(offset, doff, sizeof(long long), cudaMemcpyDeviceToHost, c->stream));
+    }
     return finish(c, flags);
 }
 

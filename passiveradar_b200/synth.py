@@ -79,3 +79,36 @@ def raw_iq(n, kind="int8", seed=11):
     if kind == "float32":
         return rng.standard_normal(2 * n).astype(np.float32)
     raise ValueError(f"unknown raw IQ kind {kind!r}")
+
+
+def offset_pair(n, offset, kind="complex64", seed=BASE_SEED + 73, snr_db=10.0):
+    """Two receiver channels of one band-limited FM-like broadcast, ``offset`` samples apart, each with its own
+    noise: ``s1[i] = s[i] + e1[i]`` and ``s2[i] = s[i + offset] + e2[i]``, so ``find_channel_offset(s1, s2, ...)``
+    finds ``offset``.  The smooth instantaneous frequency keeps the band narrow, so the correlation peak is broad
+    as on recorded data.  ``kind``: ``complex64`` (complex baseband), or ``int8`` / ``int16`` (a real band-pass
+    signal quantised as a receiver delivers raw samples)."""
+    rng = np.random.default_rng(seed)
+    total = n + abs(int(offset))
+    knots = rng.standard_normal(total // 64 + 2)
+    msg = np.interp(np.arange(total) / 64.0, np.arange(knots.size), knots)
+    real = kind in ("int8", "int16")
+    freq = (0.12 if real else 0.0) + 0.06 * msg                  # cycles per sample
+    phase = 2.0 * np.pi * np.cumsum(freq)
+    s = np.cos(phase) if real else np.exp(1j * phase)
+    a = max(0, -int(offset))
+    sigma = 10.0 ** (-snr_db / 20.0)
+
+    def noise():
+        if real:
+            return sigma * rng.standard_normal(n)
+        return sigma * (rng.standard_normal(n) + 1j * rng.standard_normal(n)) / np.sqrt(2.0)
+
+    s1 = s[a:a + n] + noise()
+    s2 = s[a + offset:a + offset + n] + noise()
+    if kind == "complex64":
+        return s1.astype(np.complex64), s2.astype(np.complex64)
+    if real:
+        scale, lim, dt = (40.0, 127, np.int8) if kind == "int8" else (4000.0, 32767, np.int16)
+        q = lambda v: np.clip(np.round(v * scale), -lim - 1, lim).astype(dt)
+        return q(s1), q(s2)
+    raise ValueError(f"unknown kind {kind!r}")
